@@ -280,15 +280,42 @@ def layer_checksum(layer, fields):
 ESDF_FIELDS = ("squared_distance_vox", "parent_direction", "is_inside", "observed", "is_site")
 
 
+def log_odds_layer(layer):
+    """{index: {"log_odds": (8,8,8) float32}} of an occupancy layer, whatever the container."""
+    return {k: {"log_odds": np.ascontiguousarray(v["log_odds"] if getattr(v, "dtype", None) is not None and v.dtype.names else v,
+                                                 dtype=np.float32)} for k, v in layer.items()}
+
+
+DUMP_MAX_BLOCKS = 2048  # per layer: 2048 ESDF blocks are 29 MB of float32, 2048 TSDF blocks 8 MB
+
+
+def dump_outputs(out_dir, projective, esdf, occupancy):
+    """Writes the map a step built as out_dir/<layer>_<field>.npy, so that two builds can be compared output for output.
+    <layer>_block_indices: every allocated block, sorted, (n, 3) float64. <layer>_sample: the positions in that list of the
+    blocks whose voxels are written (all of them, or DUMP_MAX_BLOCKS drawn with a fixed seed), float64.
+    <layer>_<field>: those blocks' voxel field, float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    if occupancy:
+        layers = (("occupancy", log_odds_layer(projective), ("log_odds",)), ("esdf", esdf, ESDF_FIELDS))
+    else:
+        layers = (("tsdf", projective, ("distance", "weight")), ("esdf", esdf, ESDF_FIELDS))
+    for name, layer, fields in layers:
+        keys = sorted(layer)
+        pick = np.arange(len(keys))
+        if len(keys) > DUMP_MAX_BLOCKS:
+            pick = np.sort(np.random.default_rng(0).choice(len(keys), DUMP_MAX_BLOCKS, replace=False))
+        np.save(os.path.join(out_dir, name + "_block_indices.npy"), np.array(keys, np.float64).reshape(-1, 3))
+        np.save(os.path.join(out_dir, name + "_sample.npy"), pick.astype(np.float64))
+        for f in fields:
+            np.save(os.path.join(out_dir, "%s_%s.npy" % (name, f)), np.array([layer[keys[i]][f] for i in pick], np.float32))
+
+
 def parity_check(m, o, occupancy=False):
     """Post-timing check, outside every timed region: the map the benchmarked pipeline just built (device-resident
     frames, asynchronous calls, ESDF wavefront overlapping the next frame's TSDF chain) against the oracle's map of
     the same sequence: allocated block sets, projective-layer bits, all five EsdfVoxel fields."""
     if occupancy:
-        def plain(layer):  # {index: (8,8,8) float32 log odds} whatever the container
-            return {k: {"log_odds": np.ascontiguousarray(v["log_odds"] if getattr(v, "dtype", None) is not None and v.dtype.names else v,
-                                                         dtype=np.float32)} for k, v in layer.items()}
-        p_gpu, p_cpu, pf = plain(m.occupancy_layer().as_dict()), plain(o.occupancy_layer()), ("log_odds",)
+        p_gpu, p_cpu, pf = log_odds_layer(m.occupancy_layer().as_dict()), log_odds_layer(o.occupancy_layer()), ("log_odds",)
     else:
         p_gpu, p_cpu, pf = m.tsdf_layer().as_dict(), o.tsdf_layer(), ("distance", "weight")
     e_gpu, e_cpu = m.esdf_layer().as_dict(), o.esdf_layer()
@@ -310,14 +337,16 @@ def run_reference(args, rank, world):
     orc.set_num_threads(cpu_threads())
 
     def step():
-        wl.oracle_map(orc, wl.frames, VOXEL)
+        return wl.oracle_map(orc, wl.frames, VOXEL)
 
     for _ in range(args.warmup):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        o = step()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, o.occupancy_layer() if wl.occupancy else o.tsdf_layer(), o.esdf_layer(), wl.occupancy)
     value = args.steps * len(wl.frames) / dt
     sample = "each step = the %d-frame step of workload %s on the host cores (same work as one GPU step of one rank)" % (len(wl.frames), wl.name)
     print(json.dumps({
@@ -350,7 +379,11 @@ def main():
     ap.add_argument("--no-merge", action="store_true", help="A/B only: ranks do not merge their block lists")
     ap.add_argument("--voxel-size", type=float, default=VOXEL,
                     help="side study only (e.g. 0.02 = the Redwood-shape config): the headline metric is quoted at 0.05")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the map the last timed step built (rank 0) as DIR/<layer>_<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -463,6 +496,9 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_max = float(t.item())
     value = world * F * args.steps / (ms_max * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, (m.occupancy_layer() if wl.occupancy else m.tsdf_layer()).as_dict(),
+                     m.esdf_layer().as_dict(), wl.occupancy)
 
     # ---- the merge on its own: device time of all-gather + union per batch (one extra, untimed step) ----
     merge_info = None

@@ -1,15 +1,19 @@
 """Builds tests/golden/threedmatch_seq01.npz from the reference's own test data
 (nvblox/tests/data/3dmatch: five 640x480 16-bit depth PNGs of seq-01 with poses, camera-intrinsics.txt, the colour image of
-frame 0) and the oracle's results on them. Run where /root/reference exists:
+frame 0) and the oracle's results on them, and tests/golden/threedmatch_seq01_sources.json: the SHA-256 of every input
+array as read from the reference's files, which tests/test_oracle_threedmatch.py checks the fixture against. Run with the root
+of an isaac_ros_nvblox checkout:
 
-    python tests/golden/make_threedmatch_fixture.py
+    python tests/golden/make_threedmatch_fixture.py <isaac_ros_nvblox checkout>
 
 The inputs are stored raw (uint16 millimetres, float32 poses parsed like parsePoseFromFile /
-parseCameraFromFile, nvblox/executables/src/datasets/3dmatch.cpp:31-75) so that the GPU box, which has no /root/reference, can
-run the same frames; the depth conversion is io::readFromPng's (nvblox/src/io/image_io.cpp:117-154):
+parseCameraFromFile, nvblox/executables/src/datasets/3dmatch.cpp:31-75) so that the tests run the same frames without the
+reference tree; the depth conversion is io::readFromPng's (nvblox/src/io/image_io.cpp:117-154):
 float(u16) * kDefaultUintDepthScaleFactor, kDefaultUintDepthScaleFactor = 1.0f / 1000.0f (nvblox/include/nvblox/io/image_io.h:32).
 The loader known answers of nvblox/tests/test_3dmatch.cpp:60-87 are asserted here and in tests/test_oracle_threedmatch.py.
 """
+import hashlib
+import json
 import os
 import sys
 
@@ -18,14 +22,17 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
-DATA = "/root/reference/nvblox_ros/nvblox_core/nvblox/tests/data/3dmatch"
+DATA = os.path.join("nvblox_ros", "nvblox_core", "nvblox", "tests", "data", "3dmatch")
 FRAMES = (0, 1, 2, 116, 422)
 OUT = os.path.join(ROOT, "tests", "golden", "threedmatch_seq01.npz")
+SOURCES = os.path.join(ROOT, "tests", "golden", "threedmatch_seq01_sources.json")
+INPUTS = ("intrinsics", "depth_u16", "poses", "color0")
 VOXEL = 0.05
 
 
-def load_reference_data(data=DATA):
+def load_reference_data(checkout):
     from PIL import Image
+    data = os.path.join(checkout, DATA)
     K = np.array([[np.float32(t) for t in line.split()] for line in open(os.path.join(data, "camera-intrinsics.txt")) if line.strip()],
                  np.float32)
     depth, poses = [], []
@@ -38,6 +45,12 @@ def load_reference_data(data=DATA):
     color0 = np.array(Image.open(os.path.join(data, "seq-01", "frame-000000.color.png")).convert("RGB"), np.uint8)
     assert color0.shape == (480, 640, 3)
     return K, np.stack(depth), np.stack(poses), color0
+
+
+def input_digests(*arrays):
+    """{input name: "dtype shape sha256"} of the arrays INPUTS names, in that order."""
+    return {k: "%s %s %s" % (a.dtype.str, "x".join(map(str, a.shape)), hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest())
+            for k, a in zip(INPUTS, arrays)}
 
 
 def depth_to_float(depth_u16):
@@ -70,7 +83,9 @@ def run_oracle(K, depth_u16, poses, color0, voxel=VOXEL):
 
 def main():
     from helpers import ESDF_FIELDS, layer_checksum
-    K, depth, poses, color0 = load_reference_data()
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    K, depth, poses, color0 = load_reference_data(sys.argv[1])
     check_loader_kats(K, depth)
     o, lists = run_oracle(K, depth, poses, color0)
     out = dict(intrinsics=K, depth_u16=depth, poses=poses, color0=color0, frames=np.array(FRAMES), voxel_size=np.float32(VOXEL),
@@ -81,6 +96,9 @@ def main():
     for i, b in enumerate(lists):
         out["blocks_%d" % i] = b
     np.savez_compressed(OUT, **out)
+    with open(SOURCES, "w") as f:
+        json.dump(input_digests(K, depth, poses, color0), f, indent=1)
+        f.write("\n")
     print("wrote", OUT, os.path.getsize(OUT), "bytes;", len(o.tsdf_layer()), "tsdf blocks; lists", [len(b) for b in lists])
 
 

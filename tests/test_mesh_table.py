@@ -1,14 +1,15 @@
 """The marching-cubes case table (isaac_ros_nvblox_b200/csrc/nvb_mc_table.h and the oracle's copy oracle/mc_table.h):
 the two copies are equal, the table satisfies the invariants of the published table (every triangle uses only edges whose two
-corners lie on opposite sides of the surface; complementary configurations have the same edges), and -- where the reference
-tree is on this machine -- every row equals the reference's (nvblox/include/nvblox/mesh/internal/impl/marching_cubes_table.h:34-333)."""
+corners lie on opposite sides of the surface; complementary configurations have the same edges), and every row equals the
+reference's (nvblox/include/nvblox/mesh/internal/impl/marching_cubes_table.h:34-333), stored as
+tests/golden/reference_mc_table.npz by tests/golden/make_reference_mc_table.py."""
 import os
 import re
 
-import pytest
+import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/nvblox_ros/nvblox_core/nvblox/include/nvblox/mesh/internal/impl/marching_cubes_table.h"
+REF = os.path.join(ROOT, "tests", "golden", "reference_mc_table.npz")
 EDGE_CORNERS = [(0, 1), (1, 2), (2, 3), (3, 0), (4, 5), (5, 6), (6, 7), (7, 4), (0, 4), (1, 5), (2, 6), (3, 7)]
 
 
@@ -39,16 +40,10 @@ def test_table_invariants():
 
 
 def test_table_equals_the_reference_table():
-    if not os.path.exists(REF):
-        pytest.skip("the reference tree is not on this machine")
-    src = open(REF).read()
-    body = src[src.index("kTriangleTable[256][16]"):]
-    body = body[body.index("{") + 1:body.index("};")]
-    ref = [[int(x) for x in re.findall(r"-?\d+", r)] for r in re.findall(r"\{([^{}]*)\}", body)]
+    g = np.load(REF)
+    ref, nt = g["triangle_table"].tolist(), g["num_triangles"].tolist()
     assert len(ref) == 256
     rows = _rows(os.path.join(ROOT, "oracle", "mc_table.h"))
     for cfg in range(256):
         assert [v for v in ref[cfg] if v >= 0] == rows[cfg], cfg
-    nt = src[src.index("kNumTrianglesTable[256]"):]
-    nt = [int(x) for x in re.findall(r"\d+", nt[nt.index("{"):nt.index("};")])]
     assert [len(r) // 3 for r in rows] == nt

@@ -1,10 +1,12 @@
 """The oracle on REFERENCE-HELD real data: the five 3DMatch frames the reference ships for its own tests
 (nvblox/tests/data/3dmatch/seq-01, real 640x480 16-bit depth with ~13 % invalid pixels, poses, intrinsics, one colour image),
 stored raw in tests/golden/threedmatch_seq01.npz by tests/golden/make_threedmatch_fixture.py.
-  * where /root/reference exists: the fixture's inputs are the reference's files, bit for bit;
+  * the fixture's inputs are the reference's files, bit for bit: their SHA-256, taken from the reference's files when the
+    fixture was made, is stored in tests/golden/threedmatch_seq01_sources.json;
   * the reference's own loader known answers (tests/test_3dmatch.cpp:60-87) hold for the fixture;
   * the oracle reproduces the committed per-frame block lists and layer checksums (TSDF + colour + ESDF).
 The CUDA path is compared with the oracle on the same frames in tests/test_gpu_bench_pipeline.py."""
+import json
 import os
 import sys
 
@@ -24,11 +26,9 @@ def fx():
 
 
 def test_fixture_inputs_are_the_reference_files(fx):
-    if not os.path.isdir(mk.DATA):
-        pytest.skip("the reference tree is not on this machine (GPU box): the committed fixture is used as is")
-    K, depth, poses, color0 = mk.load_reference_data()
-    assert np.array_equal(K, fx["intrinsics"]) and np.array_equal(depth, fx["depth_u16"])
-    assert np.array_equal(poses, fx["poses"]) and np.array_equal(color0, fx["color0"])
+    with open(mk.SOURCES) as f:
+        want = json.load(f)
+    assert mk.input_digests(*(fx[k] for k in mk.INPUTS)) == want
 
 
 def test_reference_loader_known_answers(fx):
